@@ -7,7 +7,7 @@ Workload (config 2 of BASELINE.json, the one the metric is quoted on):
   (guide sampling, model, fused scoring, backward, fused optimiser, loss read-back).
 
     python bench.py --gpus N --steps K --warmup W          # our arm  (torchrun for N > 1)
-    python bench.py --impl reference ...                   # reference arm: UNMODIFIED Pyro (baseline/_ref) on the host cores
+    python bench.py --impl reference ...                   # reference arm: UNMODIFIED Pyro (oracle/_ref) on the host cores
 
 One JSON line on stdout (rank 0).  Keys follow the driver contract; extra keys:
   roofline      dominant kernel of the measured path: algorithmic bytes per launch / its average
@@ -26,6 +26,9 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+# run from a tree that build() has completed (the build() call below then finds everything current), the
+# benchmark writes nothing into it, so that the tree may be read-only: no bytecode caches either
+sys.dont_write_bytecode = True
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -196,6 +199,20 @@ def time_steps(svi, args, steps, warmup, device, flush, sync_each=True):
     return ms, loss
 
 
+def dump_outputs(out_dir, loss):
+    """What a caller of the timed path holds after its last step: the loss it returned and every parameter
+    of the store (constrained values), as ``<out_dir>/<name>.npy`` in float32 / float64."""
+    import numpy as np
+    import pyro_b200 as pyro
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), np.asarray(loss, dtype=np.float64))
+    store = pyro.get_param_store()
+    for name in sorted(store.keys()):
+        t = store[name].detach().cpu()
+        np.save(os.path.join(out_dir, "param_%s.npy" % name),
+                t.numpy() if t.dtype == torch.float64 else t.float().numpy())
+
+
 def kernel_time_ms(fn, iters, flush):
     """Average device time of one launch sequence ``fn``: CUDA events on the launching stream
     around a replay of the sequence captured in a CUDA graph (so the Python wrapper cost of the
@@ -265,19 +282,19 @@ def roofline_for(path, X, y, particles, flush):
 
 
 class _RefPyroSVI:
-    """UNMODIFIED reference Pyro (pyro 1.9.1, pip-installed from /root/reference into baseline/_ref by
-    __graft_entry__.build(), plus the stand-in for its absent opt_einsum dependency) running the same
+    """UNMODIFIED reference Pyro (pyro 1.9.1, copied into oracle/_ref by __graft_entry__.build(),
+    plus the stand-in for its absent opt_einsum dependency) running the same
     workload through its own public API on CPU tensors: pyro.infer.SVI / Trace_ELBO(num_particles=64,
     vectorize_particles=True) / pyro.optim.ClippedAdam.  None of this repo's kernels is involved."""
 
     def __init__(self):
         from pyro_b200 import bind
         if not bind.add_reference_to_path():
-            raise RuntimeError("baseline/_ref is missing")
+            raise RuntimeError("oracle/_ref is missing")
         import pyro
         import pyro.distributions as dist
         from torch.distributions import constraints
-        assert "baseline" in pyro.__file__ and pyro.__version__.startswith("1.9")
+        assert os.path.join("oracle", "_ref") in pyro.__file__ and pyro.__version__.startswith("1.9")
         pyro.clear_param_store()
 
         def model(X, y):
@@ -307,7 +324,7 @@ class _RefPyroSVI:
 
 
 def _ref_pyro_nuts(y, sigma, warmup=100, samples=100):
-    """eight_schools through UNMODIFIED reference Pyro (baseline/_ref): pyro.infer.MCMC(pyro.infer.NUTS(model)),
+    """eight_schools through UNMODIFIED reference Pyro (oracle/_ref): pyro.infer.MCMC(pyro.infer.NUTS(model)),
     one chain on the host; leapfrogs counted at pyro.ops.integrator.potential_grad (one call per leapfrog,
     pyro/ops/integrator.py:45-65).  None when the reference is not importable."""
     try:
@@ -317,7 +334,7 @@ def _ref_pyro_nuts(y, sigma, warmup=100, samples=100):
         import pyro
         import pyro.distributions as dist
         import pyro.ops.integrator as integ
-        assert "baseline" in pyro.__file__
+        assert os.path.join("oracle", "_ref") in pyro.__file__
     except Exception:  # noqa: BLE001
         return None
 
@@ -638,7 +655,11 @@ def main():
     ap.add_argument("--cpu-steps", type=int, default=4)
     ap.add_argument("--no-nuts", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the config 3 / config 5 sections")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the loss and parameters of the last step as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     a.warmup = max(a.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -647,10 +668,10 @@ def main():
     if a.impl == "reference":
         if rank != 0:
             return
-        steps = min(a.steps, 20)
+        steps = a.steps
         v, ms, threads, loss = cpu_reference(steps, min(a.warmup, 2))
         kind = cpu_reference.kind
-        what = ("pyro.infer.SVI.step of unmodified Pyro (baseline/_ref)" if kind == "reference"
+        what = ("pyro.infer.SVI.step of unmodified Pyro (oracle/_ref)" if kind == "reference"
                 else "oracle/svi.py LogisticSVIMatmul")
         out = {"impl": "reference", "metric": METRIC, "value": round(v, 4), "unit": UNIT, "n_gpus": a.gpus,
                "steps": steps, "warmup": min(a.warmup, 2), "ms_per_step": round(ms, 3),
@@ -710,6 +731,8 @@ def main():
         time.sleep(0.15)
     ms, loss = time_steps(svi, step_args, a.steps, a.warmup + 2, dev, flush)
     torch.cuda.synchronize(dev)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, loss)
     if world > 1:
         dist.barrier()
     total_ms = torch.tensor([sum(ms)], device=dev, dtype=torch.float64)
@@ -859,7 +882,7 @@ def main():
         out["cpu_baseline"] = {"value": round(v, 4), "unit": UNIT, "cores": threads, "kind": cpu_reference.kind,
                                "sample": "%d full-size steps (N=1e6, P=64) of %s, torch CPU ops, the fastest of "
                                          "several host thread counts" % (
-                                             a.cpu_steps, "pyro.infer.SVI.step of unmodified Pyro (baseline/_ref)"
+                                             a.cpu_steps, "pyro.infer.SVI.step of unmodified Pyro (oracle/_ref)"
                                              if cpu_reference.kind == "reference" else "oracle/svi.py LogisticSVIMatmul"),
                                "ms_per_step": round(cms, 2)}
         if not a.no_nuts:

@@ -1,7 +1,7 @@
 """Binding of the native kernels into UNMODIFIED reference Pyro (the stub a maintainer would add).
 
-``import pyro`` must already work (the reference tree on ``sys.path``; on the GPU box that is
-``baseline/_ref`` + the ``opt_einsum`` stand-in, see :func:`add_reference_to_path`).  Nothing in Pyro is
+``import pyro`` must already work (the reference tree on ``sys.path``; in this repository's tests that is
+``oracle/_ref`` + the ``opt_einsum`` stand-in, see :func:`add_reference_to_path`).  Nothing in Pyro is
 patched; every object below plugs into a seam the reference already exposes (SURVEY.md 8b):
 
 =====================  ==========================================================================
@@ -41,10 +41,10 @@ _ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def add_reference_to_path():
-    """Make ``import pyro`` resolve to the vendored, unmodified reference (``baseline/_ref``, installed by
-    ``__graft_entry__.build()`` with pip from /root/reference) plus the ~30-line stand-in for its
-    absent ``opt_einsum`` dependency.  Returns True if both are present."""
-    ref = os.path.join(_ROOT, "baseline", "_ref")
+    """Make ``import pyro`` resolve to the vendored, unmodified reference (``oracle/_ref``, installed by
+    ``__graft_entry__.build()`` from the reference source tree, oracle/reference_pyro.py) plus the ~30-line
+    stand-in for its absent ``opt_einsum`` dependency.  Returns True if both are present."""
+    ref = os.path.join(_ROOT, "oracle", "_ref")
     shim = os.path.join(_ROOT, "tests", "golden", "opt_einsum_standin")
     if not os.path.isdir(os.path.join(ref, "pyro")):
         return False

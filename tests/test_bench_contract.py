@@ -19,10 +19,10 @@ def test_reference_arm_prints_one_json_line():
     assert d["impl"] == "reference" and d["metric"] == "svi_steps_per_sec" and d["unit"] == "steps/s"
     assert d["higher_is_better"] is True and d["value"] > 0 and d["n_gpus"] == 1
     assert d["config"]["workload"].startswith("bayesian_logistic_regression_svi N=1e6 D=32")
-    # unmodified Pyro when baseline/_ref is vendored (the build container and the GPU box), else the oracle port
+    # unmodified Pyro when oracle/_ref is vendored, else the oracle port
     assert d["cpu_baseline"]["kind"] == "reference" or d["cpu_baseline"]["kind"].startswith("port")
     assert d["cpu_baseline"]["cores"] >= 1
-    if os.path.isdir(os.path.join(ROOT, "baseline", "_ref", "pyro")):
+    if os.path.isdir(os.path.join(ROOT, "oracle", "_ref", "pyro")):
         assert d["cpu_baseline"]["kind"] == "reference" and "unmodified Pyro" in d["cpu_baseline"]["sample"]
     assert d["e2e"] == {"value": d["value"], "unit": "steps/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 

@@ -1,15 +1,12 @@
 """The binding of INTEGRATION.md executed against UNMODIFIED reference Pyro (pyro 1.9.1 from
-``baseline/_ref`` -- pip-installed from /root/reference by ``__graft_entry__.build()`` -- or from
-/root/reference itself in the build container): models and guides are written with ``import pyro``;
+``oracle/_ref``, copied by ``__graft_entry__.build()`` from the reference source tree,
+oracle/reference_pyro.py; without it these tests skip): models and guides are written with ``import pyro``;
 ``pyro.infer.SVI`` / ``pyro.infer.MCMC`` drive them; the kernels enter through the seams of SURVEY.md 8b
 (``loss=``, ``optim=``, ``potential_fn=``, ``kernel=``).
 
 Every scenario runs twice: in the CPU tier with the native seams replaced by the oracle-backed stand-ins
 (host logic only) and in the ``-m gpu`` tier through the real kernels.  Reference numbers are the
 goldens recorded from the same unmodified Pyro (tests/golden/make_golden.py)."""
-import os
-import sys
-
 import numpy as np
 import pytest
 import torch
@@ -17,17 +14,11 @@ from torch.distributions import constraints
 
 from conftest import EMULATE, load_npz
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
 
 def _import_pyro():
     from pyro_b200 import bind
     if not bind.add_reference_to_path():
-        if os.path.isdir("/root/reference/pyro"):
-            sys.path.insert(0, os.path.join(ROOT, "tests", "golden", "opt_einsum_standin"))
-            sys.path.insert(0, "/root/reference")
-        else:
-            pytest.skip("reference Pyro is not vendored (baseline/_ref missing)")
+        pytest.skip("reference Pyro is not vendored (oracle/_ref missing; see oracle/reference_pyro.py)")
     import pyro
     assert pyro.__version__.startswith("1.9"), pyro.__version__
     assert "pyro_b200" not in (pyro.__file__ or "")
