@@ -106,14 +106,10 @@ typedef struct {
                                     reference's small fixtures) */
 #define B2_FLAG_GLM_FP32 2       /* b2_glm_bernoulli_logits: fp32 SIMT contractions instead of the
                                     tensor-core path */
-#define B2_FLAG_GLM_TF32 8       /* b2_glm_bernoulli_logits: single-pass TF32 logits (opt-in, ~1e-3
-                                    relative per logit) instead of the default 3xTF32 split */
 #define B2_FLAG_GLM_3XTF32 32    /* b2_glm_bernoulli_logits: split X as well as W (every logit exact to
                                     ~1e-6; the default splits W only, see below) */
-#define B2_FLAG_GLM_BF16_GRAD 64 /* b2_glm_bernoulli_logits (opt-in): gradient contraction in BF16 on MN-major
-                                    operands -- 10 % faster, operand rounding 2^-9 (see below) */
-#define B2_FLAG_GLM_MMA_SYNC 16  /* b2_glm_bernoulli_logits: the legacy mma.sync kernel (single-pass
-                                    TF32) instead of the tcgen05/TMA kernel */
+/* bits 8, 16 and 64 are retired (they selected removed GLM kernel variants); b2_glm_bernoulli_logits
+   rejects them with B2_ERR_BAD_SHAPE */
 
 /*
  * b2_site_score -- fused log_prob + score of one sample site for an elementwise family.
@@ -273,17 +269,17 @@ int b2_elbo_combine(const void* const* terms, const double* coeffs, int n, int d
  * X: [N,D] row-major fp32 (16-byte aligned), D in {4, 8, 16, 32}; W: [P,D]; b: [P] (nullable);
  * y: [N] fp32.
  * out_total (nullable): scalar, (=|+=) sum_coeff * scale * SUM_p sum_p[p].
- * For D == 32 the two contractions run on the tcgen05 tensor cores out of TMA-staged tiles with
- * TMEM accumulators (glm_tc.cu).  Default precision: W is split hi + lo (two TF32 MMAs per k-step), which
- * removes the only error that is COHERENT over rows (a rounded W shifts every row's logit the same way
- * and survives the N-term sums); X and g = y - sigmoid are rounded to nearest TF32 (incoherent, averages
- * as 1/sqrt(N)): sum_p, dW, db agree with an fp64 evaluation to ~1e-6 / ~1e-5 relative at N = 1e6.
- * B2_FLAG_GLM_BF16_GRAD (opt-in): the gradient contraction in BF16 on MN-major operands (no transposition
- * pass, half the MMAs): 90 instead of 100 us at N = 1e6; operand rounding 2^-9, unbiased -- 3e-5 of the largest
- * entry on dW for generic W, but a noise floor of ~1e-3 sqrt(N) that shows when the gradient itself is ~sqrt(N)
- * (balanced data, near a stationary point), which is why it is not the default.
- * B2_FLAG_GLM_3XTF32: X split as well (every logit fp32-exact); B2_FLAG_GLM_TF32: single-pass TF32;
- * B2_FLAG_GLM_MMA_SYNC: the round-1 mma.sync kernel; B2_FLAG_GLM_FP32: the fp32 SIMT kernel.
+ * flags: B2_FLAG_ACCUMULATE_SUM, B2_FLAG_GLM_FP32, B2_FLAG_GLM_3XTF32; any other bit -> B2_ERR_BAD_SHAPE.
+ * Kernel choice:
+ *   - the exact fp32 SIMT kernel when B2_FLAG_GLM_FP32 is set, D != 32, y is not 16-byte aligned,
+ *     N >= 2^31, or N < 8192 without B2_FLAG_GLM_3XTF32;
+ *   - otherwise the tcgen05 tensor-core kernel, which runs both contractions out of TMA-staged tiles with
+ *     TMEM accumulators (glm_tc.cu).  W is split hi + lo (two TF32 MMAs per k-step), which removes the
+ *     only error that is COHERENT over rows (a rounded W shifts every row's logit the same way and
+ *     survives the N-term sums); g = y - sigmoid is rounded to nearest TF32.  X is split hi + lo as well
+ *     (every logit fp32-exact) when B2_FLAG_GLM_3XTF32 is set or N < 65536; above that it is rounded to
+ *     nearest TF32 (incoherent, averages as 1/sqrt(N)): sum_p, dW, db agree with an fp64 evaluation to
+ *     ~1e-6 / ~1e-5 relative at N = 1e6.
  * workspace: b2_glm_workspace() bytes, zero-initialised ONCE by the caller (its first 256 bytes
  * hold a ticket counter that the library leaves zeroed).  Two launches: the streaming kernel
  * and a finish kernel that sums the CTA partials in a fixed order (deterministic).

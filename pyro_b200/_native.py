@@ -20,10 +20,7 @@ B2_F32, B2_F64, B2_I64, B2_U8 = 0, 1, 2, 3
 B2_FLAG_ACCUMULATE_SUM = 1
 B2_FLAG_GLM_FP32 = 2
 B2_FLAG_SITE_LARGE = 4
-B2_FLAG_GLM_TF32 = 8
-B2_FLAG_GLM_MMA_SYNC = 16
 B2_FLAG_GLM_3XTF32 = 32
-B2_FLAG_GLM_BF16_GRAD = 64
 FORCE_LARGE_SITE_KERNELS = False   # tests: score small fixtures with the multi-CTA kernels too
 B2_ERR_UNSUPPORTED_REDUCTION = -6
 

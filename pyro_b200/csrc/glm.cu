@@ -185,14 +185,10 @@ __global__ void __launch_bounds__(256) glm_finish_kernel(const float* __restrict
   }
 }
 
-// tensor-core variant (glm_mma.cu)
-int glm_mma_grid_x(int64_t N);
-void launch_glm_mma(const float* X, const float* y, const float* W, const float* b, int64_t N, int P,
-                    float* partials, int gx, cudaStream_t s);
 // tcgen05 + TMA variant (glm_tc.cu)
 int glm_tc_grid_x(int64_t N);
 int launch_glm_tc(const float* X, const float* y, const float* W, const float* b, int64_t N, int P,
-                  float* partials, int gx, int mode, cudaStream_t s);
+                  float* partials, int gx, bool split_x, cudaStream_t s);
 
 inline int glm_grid_x(int64_t N) {
   const int64_t ntiles = (N + kGlmTileRows - 1) / kGlmTileRows;
@@ -219,31 +215,26 @@ extern "C" int b2_glm_bernoulli_logits(const float* X, const float* y, const flo
                                        void* stream) {
   if (!X || !y || !W) return B2_ERR_NULL;
   if (N <= 0 || P <= 0) return B2_ERR_BAD_SHAPE;
+  // an unknown bit is refused, not ignored: a caller asking for a kernel variant must not silently get another
+  if (flags & ~(B2_FLAG_ACCUMULATE_SUM | B2_FLAG_GLM_FP32 | B2_FLAG_GLM_3XTF32)) return B2_ERR_BAD_SHAPE;
   if (reinterpret_cast<uintptr_t>(X) % 16 != 0) return B2_ERR_BAD_SHAPE;
   if (!workspace || workspace_bytes < b2_glm_workspace(N, D, P)) return B2_ERR_WORKSPACE;
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   // below 8 Ki rows the single-pass TF32 gradient contraction has not averaged its operand rounding
   // (2^-12 relative per term) below the fp32 tolerance yet: those sizes take the exact fp32 SIMT kernel
-  // unless a tensor-core variant is asked for explicitly
-  const bool forced_tc = flags & (B2_FLAG_GLM_TF32 | B2_FLAG_GLM_3XTF32 | B2_FLAG_GLM_MMA_SYNC | B2_FLAG_GLM_BF16_GRAD);
-  const bool use_tensor = (D == 32) && !(flags & B2_FLAG_GLM_FP32) && (N >= 8192 || forced_tc);
-  const bool use_tc = use_tensor && !(flags & B2_FLAG_GLM_MMA_SYNC) &&
+  // unless B2_FLAG_GLM_3XTF32 asks for the tensor cores explicitly; the TMA loads need a 16-byte aligned y
+  // and 32-bit row coordinates
+  const bool use_tc = (D == 32) && !(flags & B2_FLAG_GLM_FP32) && (N >= 8192 || (flags & B2_FLAG_GLM_3XTF32)) &&
                       reinterpret_cast<uintptr_t>(y) % 16 == 0 && N < ((int64_t)1 << 31);
-  const bool use_mma = use_tensor && !use_tc;
-  const int gx = use_tc ? glm_tc_grid_x(N) : (use_mma ? glm_mma_grid_x(N) : glm_grid_x(N));
+  const int gx = use_tc ? glm_tc_grid_x(N) : glm_grid_x(N);
   dim3 grid((unsigned)gx, (unsigned)((P + kGlmParticles - 1) / kGlmParticles), 1);
   unsigned int* ticket = reinterpret_cast<unsigned int*>(workspace);
   float* partials = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + 256);
   if (use_tc) {
-    // default: W split; below 64 Ki rows the incoherent X rounding has not averaged out yet -> full 3xTF32
-    // B2_FLAG_GLM_BF16_GRAD (opt-in): BF16 gradient contraction on MN-major operands (MODE 3)
-    const int mode = (flags & B2_FLAG_GLM_TF32) ? 0
-                     : ((flags & B2_FLAG_GLM_BF16_GRAD) ? 3
-                        : (((flags & B2_FLAG_GLM_3XTF32) || N < 65536) ? 2 : 1));
-    const int rc = launch_glm_tc(X, y, W, b, N, P, partials, gx, mode, s);
+    // W split by default; below 64 Ki rows the incoherent X rounding has not averaged out yet -> X split too
+    const bool split_x = (flags & B2_FLAG_GLM_3XTF32) || N < 65536;
+    const int rc = launch_glm_tc(X, y, W, b, N, P, partials, gx, split_x, s);
     if (rc != 0) return rc;
-  } else if (use_mma) {
-    launch_glm_mma(X, y, W, b, N, P, partials, gx, s);
   } else
   switch (D) {
     case 4: glm_bernoulli_kernel<4><<<grid, 256, 0, s>>>(X, y, W, b, N, P, partials); break;

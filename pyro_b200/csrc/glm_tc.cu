@@ -10,12 +10,11 @@
 // Per 128-row tile (one persistent CTA per SM, tiles round-robin over CTAs):
 //
 //   GEMM 1   D1[n, p] = sum_d X[n, d] W[p, d] + b[p]      M = 128 rows, N = 64 particles, K = 32
-//            default (MODE 1): W split hi + lo, two TF32 MMAs per k-step -- the rounding of W is the only
-//            error of a TF32 GEMM 1 that is COHERENT over rows (it shifts all N logits of a particle the
-//            same way and survives the N-term sums); X is rounded to nearest in place (incoherent,
-//            averages as 1/sqrt(N)).  MODE 2 splits X as well (every logit exact to ~1e-6), MODE 0 is
-//            single-pass TF32.  fp32 accumulation in TMEM; the bias enters through one more MMA
-//            (A = ones, B = [b_hi, b_lo, 0...]).
+//            W split hi + lo, two TF32 MMAs per k-step -- the rounding of W is the only error of a TF32
+//            GEMM 1 that is COHERENT over rows (it shifts all N logits of a particle the same way and
+//            survives the N-term sums); X is rounded to nearest in place (incoherent, averages as
+//            1/sqrt(N)).  SPLIT_X splits X as well (every logit exact to ~1e-6).  fp32 accumulation in
+//            TMEM; the bias enters through one more MMA (A = ones, B = [b_hi, b_lo, 0...]).
 //   epilogue sixteen warps tcgen05.ld the 128 x 64 logits (thread = row, 16 particles each), evaluate
 //            lp = y*l - softplus(l), g = y - sigmoid(l) (3 MUFU + ~12 FMA-pipe ops per element, in
 //            batches of 8 so the MUFU latency is covered inside the warp), keep the per-particle lp sums
@@ -28,7 +27,7 @@
 //
 // TF32 MN-major operands only exist in the 32-byte-atom swizzle, so instead of re-reading the X tile
 // in a second layout, four "split" warps transform each TMA tile once: RN-rounded X in place (plus X_lo
-// in MODE 2) for GEMM 1 and the transposed X^T[d, n] for GEMM 2.  All operand tiles are K-major
+// with SPLIT_X) for GEMM 1 and the transposed X^T[d, n] for GEMM 2.  All operand tiles are K-major
 // SWIZZLE_128B, the layout TMA writes natively.
 //
 // Warp roles (704 threads): warp 0 TMA producer, warp 1 MMA issuer + TMEM owner (the whole warp walks
@@ -47,9 +46,7 @@
 //
 // Determinism: every CTA writes its partials once; glm_finish_kernel adds them in a fixed order.
 #include <cuda.h>
-#include <cuda_bf16.h>
 #include <cuda/std/type_traits>
-#include <stdlib.h>
 
 #include "b2_common.cuh"
 
@@ -72,32 +69,25 @@ constexpr uint32_t kGBuf = 4 * kP * 128;                      // g^T: [kb 4][p 6
 constexpr uint32_t kXtBlock = (kD + 8) * 128;                 // X^T k-block: 32 rows of d + 8 rows of ones
 constexpr uint32_t kXtStage = 4 * kXtBlock;                   // 20 KB
 
-// MODE 0: single-pass TF32 logits.  MODE 1 (default): W split hi/lo -- the rounding error of W is the
-// only COHERENT error of a TF32 GEMM 1 (it is the same for all rows, so it does not average out over
-// the N-term sums); X is rounded to nearest in place (incoherent, averages as 1/sqrt(N)).
-// MODE 2: full 3xTF32 (X split as well): every logit exact to ~1e-6, at the price of a shallower TMA
-// ring (the X_lo tiles take the shared memory of two X stages).
-// MODE 3: logits as MODE 1; GEMM 2 in BF16 (kind::f16, K = 16 per instruction) on MN-major operands -- g and
-// X keep their natural [row][column] layout (no transposition pass, vector stores), half the bytes, half the
-// MMAs.  Operand rounding 2^-9 (round to nearest, unbiased): 3e-5 of the largest entry of dW at N = 1e6 for
-// generic W, but a noise floor of ~1e-3 sqrt(N) that matters when the gradient itself is O(sqrt(N)); opt-in
-// (B2_FLAG_GLM_BF16_GRAD), 90 us instead of 100 us.
-template <int MODE>
+// Precision of GEMM 1 (the logits).  Default (SPLIT_X = false): W split hi/lo -- the rounding error of W
+// is the only COHERENT error of a TF32 GEMM 1 (it is the same for all rows, so it does not average out
+// over the N-term sums); X is rounded to nearest in place (incoherent, averages as 1/sqrt(N)).
+// SPLIT_X: full 3xTF32 (X split as well): every logit exact to ~1e-6, at the price of a shallower TMA
+// ring (the X_lo tiles take the shared memory of two X stages).  Taken below 64 Ki rows, where the
+// incoherent X rounding has not averaged out yet.
+template <bool SPLIT_X>
 struct Layout {
-  static constexpr bool kBf16 = (MODE == 3);
-  static constexpr int kStagesX = (MODE == 2) ? 2 : 4;             // TMA ring: X tile (hi in place) + y
-  static constexpr int kStagesL = (MODE == 2) ? 2 : 0;             // X_lo ring
+  static constexpr int kStagesX = SPLIT_X ? 2 : 4;                 // TMA ring: X tile (hi in place) + y
+  static constexpr int kStagesL = SPLIT_X ? 2 : 0;                 // X_lo ring
   static constexpr int kStagesT = 3;                               // GEMM 2 B-operand (+ y) ring: split pass -> GEMM 2
                                                                    // (>= 3: GEMM 1 runs two tiles ahead)
-  static constexpr uint32_t kXtStage = kBf16 ? kTile : b2::tc::kXtStage;   // bf16 [128 n][64 cols] = 16 KB
-  static constexpr uint32_t kGBuf = kBf16 ? kTile : b2::tc::kGBuf;         // bf16 [128 n][64 p]   = 16 KB
   static constexpr uint32_t OFF_X = 0;
   static constexpr uint32_t OFF_XLO = OFF_X + kStagesX * kTile;
   static constexpr uint32_t OFF_XT = OFF_XLO + kStagesL * kTile;   // [stage][kb 4][d 32 + 8 ones][32 n] fp32
   static constexpr uint32_t OFF_G = OFF_XT + kStagesT * kXtStage;
   // the g buffers double as the [128][65] fp32 scratch of the final reduction (33 280 bytes)
-  static constexpr uint32_t kGRegion = (2 * kGBuf > 34816u) ? 2 * kGBuf : 34816u;
-  static constexpr uint32_t OFF_WHI = OFF_G + kGRegion;           // [p 64][32 d] SW128, 8 KB
+  static_assert(2 * kGBuf >= 128 * 65 * 4, "reduction scratch");
+  static constexpr uint32_t OFF_WHI = OFF_G + 2 * kGBuf;           // [p 64][32 d] SW128, 8 KB
   static constexpr uint32_t OFF_WLO = OFF_WHI + 8192;
   static constexpr uint32_t OFF_WB = OFF_WLO + 8192;               // bias tile (k = 0: b_hi, k = 1: b_lo)
   static constexpr uint32_t OFF_ONES = OFF_WB + 8192;              // 4 KB of 1.0f (no-swizzle operand)
@@ -106,15 +96,14 @@ struct Layout {
   static constexpr uint32_t OFF_BAR = OFF_YX + kStagesX * 512;
   static constexpr uint32_t kSmemBytes = OFF_BAR + 256 + 1024;     // + slack for the 1024-byte alignment
 };
-static_assert(Layout<1>::kSmemBytes <= 232448 && Layout<2>::kSmemBytes <= 232448 &&
-                  Layout<3>::kSmemBytes <= 232448, "shared memory budget");
+static_assert(Layout<false>::kSmemBytes <= 232448 && Layout<true>::kSmemBytes <= 232448, "shared memory budget");
 
 // barrier slots (8 bytes each)
 enum : int {
   BAR_XFULL = 0,                         // [kMaxStagesX] TMA landed
   BAR_XREADY = BAR_XFULL + kMaxStagesX,  // [kMaxStagesX] split pass done
   BAR_XEMPTY = BAR_XREADY + kMaxStagesX, // [kMaxStagesX] GEMM 1 finished reading the X tile
-  BAR_LEMPTY = BAR_XEMPTY + kMaxStagesX, // [2] GEMM 1 finished reading X_lo (MODE 2)
+  BAR_LEMPTY = BAR_XEMPTY + kMaxStagesX, // [2] GEMM 1 finished reading X_lo (SPLIT_X)
   BAR_TEMPTY = BAR_LEMPTY + 2,           // [kStagesT] GEMM 2 finished reading X^T
   BAR_D1FULL = BAR_TEMPTY + kMaxStagesT, // [2]
   BAR_D1EMPTY = BAR_D1FULL + 2,          // [2]
@@ -190,20 +179,6 @@ __host__ __device__ constexpr uint32_t idesc_tf32(int M, int N) {
   return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 
-// kind::f16 with BF16 operands (format code 1), both MN-major (bits 15 / 16), fp32 accumulate
-__host__ __device__ constexpr uint32_t idesc_bf16_mn(int M, int N) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) | ((uint32_t)(N >> 3) << 17) |
-         ((uint32_t)(M >> 4) << 24);
-}
-__device__ __forceinline__ void mma_bf16(uint32_t d_tmem, uint64_t a, uint64_t b, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(a), "l"(b), "r"(idesc), "r"(acc)
-      : "memory");
-}
-
 __device__ __forceinline__ void mma_tf32(uint32_t d_tmem, uint64_t a, uint64_t b, uint32_t idesc, uint32_t acc) {
   asm volatile(
       "{\n\t.reg .pred p;\n\t"
@@ -249,19 +224,7 @@ __device__ __forceinline__ float tf32_rn(float x) {
 
 // B elements at once, stage by stage: the MUFU results are consumed a whole stage (>= B instructions)
 // after they were issued, so their latency is covered inside the warp instead of by warp switching.
-// g[n][p] as bf16, natural layout (MN-major A operand of the BF16 GEMM 2): 8 values = one 16-byte chunk
-__device__ __forceinline__ void store_g_bf16(uint8_t* gt, int r, int chunk, const float (&g)[8]) {
-  __nv_bfloat162 a = __floats2bfloat162_rn(g[0], g[1]), b = __floats2bfloat162_rn(g[2], g[3]);
-  __nv_bfloat162 c = __floats2bfloat162_rn(g[4], g[5]), d = __floats2bfloat162_rn(g[6], g[7]);
-  uint4 v;
-  v.x = *reinterpret_cast<uint32_t*>(&a);
-  v.y = *reinterpret_cast<uint32_t*>(&b);
-  v.z = *reinterpret_cast<uint32_t*>(&c);
-  v.w = *reinterpret_cast<uint32_t*>(&d);
-  *reinterpret_cast<uint4*>(gt + r * 128 + ((chunk ^ (r & 7)) << 4)) = v;
-}
-
-template <bool MASK, int B, bool RAW = false>
+template <bool MASK, int B>
 __device__ __forceinline__ void epi_batch(const uint32_t* lr, float y, float vw, float* acc, float* g) {
   float e[B], den[B], inv[B], lg[B];
 #pragma unroll
@@ -293,25 +256,19 @@ __device__ __forceinline__ void epi_batch(const uint32_t* lr, float y, float vw,
     } else {
       acc[j] = fmaf(lg[j], -0.6931471805599453f, acc[j]);
     }
-    g[j] = RAW ? gg : tf32_rn(gg);
+    g[j] = tf32_rn(gg);
   }
 }
 
-template <int MODE>
+template <bool SPLIT_X>
 __global__ void __launch_bounds__(kThreads, 1)
 glm_bernoulli_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_y,
                         const float* __restrict__ W, const float* __restrict__ bvec, int64_t N, int P,
-                        float* __restrict__ partials, long long* __restrict__ trace) {
+                        float* __restrict__ partials) {
   pdl_enter();   // lets glm_finish_kernel be resident (blocked in its griddepcontrol.wait) before this kernel ends
-  using L = Layout<MODE>;
-  // optional event trace of CTA (0, 0): trace[it * 16 + k] = SM clock of event k of tile it (first 64 tiles)
-  const bool tr = (trace != nullptr) && blockIdx.x == 0 && blockIdx.y == 0;
-#define TRACE(it_, k_) do { if (tr && (it_) < 64) trace[(it_) * 16 + (k_)] = clock64(); } while (0)
+  using L = Layout<SPLIT_X>;
   constexpr int SX = L::kStagesX;
   constexpr int kStagesT = L::kStagesT;
-  constexpr bool BF = L::kBf16;              // GEMM 2 in BF16 on MN-major operands
-  constexpr int LM = BF ? 1 : MODE;          // precision mode of the logits (GEMM 1)
-  constexpr uint32_t kXtStage = L::kXtStage, kGBuf = L::kGBuf;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw = smem_u32(smem_raw);
   const uint32_t base = (raw + 1023u) & ~1023u;
@@ -360,7 +317,7 @@ glm_bernoulli_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
       const int p = e >> 5, d = e & 31;
       const int gp = slab * kP + p;
       const float w = (gp < P) ? W[(int64_t)gp * kD + d] : 0.f;
-      const float hi = (LM >= 1) ? tf32_trunc(w) : tf32_rn(w);
+      const float hi = tf32_trunc(w);
       const int off = p * 32 + ((((d >> 2) ^ (p & 7)) << 2) | (d & 3));   // float index, 128B swizzle
       whi[off] = hi;
       wlo[off] = w - hi;
@@ -374,21 +331,10 @@ glm_bernoulli_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
     }
     float* ones = reinterpret_cast<float*>(sm + L::OFF_ONES);
     for (int e = tid; e < 1024; e += kThreads) ones[e] = 1.f;
-    if (!BF) {
-      // rows 32..39 of every X^T k-block are ones: GEMM 2 then yields db in columns 32..39 of D2
-      for (int e = tid; e < kStagesT * 4 * 256; e += kThreads) {
-        const int blk = e >> 8, w = e & 255;
-        reinterpret_cast<float*>(sm + L::OFF_XT + blk * kXtBlock + kD * 128)[w] = 1.f;
-      }
-    } else {
-      // bf16 B operand [128 n][64 columns]: columns 0..31 = x (split pass), column 32 = 1 (-> db in column
-      // 32 of D2), columns 33..63 = 0.  The constant chunks 4..7 of every row are written once here
-      // (16-byte chunk c of row n sits at chunk position c ^ (n & 7): 128-byte swizzle).
-      for (int e = tid; e < kStagesT * kRows * 4; e += kThreads) {
-        const int stg = e / (kRows * 4), rr = (e / 4) % kRows, c = 4 + (e & 3);
-        uint4 v = make_uint4(c == 4 ? 0x00003f80u : 0u, 0u, 0u, 0u);   // bf16 1.0 = 0x3f80 in element 0
-        *reinterpret_cast<uint4*>(sm + L::OFF_XT + stg * kXtStage + rr * 128 + ((c ^ (rr & 7)) << 4)) = v;
-      }
+    // rows 32..39 of every X^T k-block are ones: GEMM 2 then yields db in columns 32..39 of D2
+    for (int e = tid; e < kStagesT * 4 * 256; e += kThreads) {
+      const int blk = e >> 8, w = e & 255;
+      reinterpret_cast<float*>(sm + L::OFF_XT + blk * kXtBlock + kD * 128)[w] = 1.f;
     }
   }
   fence_proxy_async();
@@ -404,7 +350,6 @@ glm_bernoulli_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
         const int sx = it % SX, ux = it / SX;
         const int64_t tile = blockIdx.x + (int64_t)it * gridDim.x;
         mbar_wait(bar(BAR_XEMPTY + sx), (ux & 1) ^ 1);
-        TRACE(it, 0);
         mbar_expect_tx(bar(BAR_XFULL + sx), kXStage);
         tma_load_2d(base + L::OFF_X + sx * kTile, &map_x, 0, (int)(tile * kRows), bar(BAR_XFULL + sx));
         tma_load_1d(base + L::OFF_YX + sx * 512, &map_y, (int)(tile * kRows), bar(BAR_XFULL + sx));
@@ -428,7 +373,7 @@ glm_bernoulli_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
     const uint64_t d_xl0 = desc_sw128(base + L::OFF_XLO);
     const uint64_t d_g0 = desc_sw128(base + L::OFF_G);
     const uint64_t d_xt0 = desc_sw128(base + L::OFF_XT);
-    constexpr int kG1 = (LM == 2) ? 12 : (LM == 1 ? 8 : 4);   // data MMAs of GEMM 1
+    constexpr int kG1 = SPLIT_X ? 12 : 8;                        // data MMAs of GEMM 1
     constexpr int n_g1 = kG1 + 1;                                 // + the bias MMA (a zero tile without bias)
 
     // i-th MMA of GEMM 1 (i is a compile-time constant after unrolling); d1 / ax / al: accumulator and
@@ -447,7 +392,7 @@ glm_bernoulli_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
     auto g1_commit = [&](int it) {
       tc_commit(bar(BAR_D1FULL + (it & 1)));
       tc_commit(bar(BAR_XEMPTY + it % SX));
-      if (LM == 2) tc_commit(bar(BAR_LEMPTY + (it & 1)));
+      if (SPLIT_X) tc_commit(bar(BAR_LEMPTY + (it & 1)));
     };
     auto g1_wait = [&](int it) {
       mbar_wait(bar(BAR_XREADY + it % SX), (it / SX) & 1);
@@ -467,23 +412,6 @@ glm_bernoulli_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
       const uint64_t db0 = d_xt0 + (uint64_t)((uint32_t)st * (kXtStage >> 4));
       const uint32_t acc0 = j > 0 ? 1u : 0u;
       int gi = 0;
-      if (BF) {
-        // 8 MMAs of K = 16 rows (2048 bytes of both MN-major tiles per step), one accumulator
-        constexpr uint32_t id2b = idesc_bf16_mn(64, 64);
-#pragma unroll
-        for (int k = 0; k < 8; ++k) {
-          mma_bf16(tmem + kColD2, da0 + (uint64_t)(k * 128), db0 + (uint64_t)(k * 128), id2b, k > 0 ? 1u : acc0);
-          if (WITH_G1) {
-            const int upto = ((k + 1) * n_g1 + 7) >> 3;
-#pragma unroll
-            for (int q = 0; q < 3; ++q)
-              if (gi < upto) {
-                g1_mma(gi, d1, ax, al);
-                ++gi;
-              }
-          }
-        }
-      } else {
 #pragma unroll
       for (int sstep = 0; sstep < 4; ++sstep) {
 #pragma unroll
@@ -502,7 +430,6 @@ glm_bernoulli_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
           }
         }
       }
-      }
       if (WITH_G1) g1_commit(it);
       tc_commit(bar(BAR_TEMPTY + st));
       tc_commit(bar(BAR_GEMPTY + bj));
@@ -510,7 +437,6 @@ glm_bernoulli_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
     // prologue: GEMM 1 of the first two tiles
     for (int it = 0; it < 2 && it < nt; ++it) {
       g1_wait(it);
-      if (lane == 0) TRACE(it, 1);
       tc_fence_after();
       if (elect_one()) {
         const uint32_t d1 = tmem + kColD1 + (uint32_t)(it & 1) * 64u;
@@ -521,20 +447,17 @@ glm_bernoulli_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
         g1_commit(it);
       }
       __syncwarp();
-      if (lane == 0) TRACE(it, 3);
     }
     for (int j = 0; j < nt; ++j) {
       const bool has_g1 = (j + 2 < nt);
       if (has_g1) g1_wait(j + 2);                      // long satisfied: split pass / epilogue of older tiles
       mbar_wait(bar(BAR_GFULL + (j & 1)), (j >> 1) & 1);   // epilogue of tile j has written g^T
-      if (lane == 0) TRACE(j, 4);
       tc_fence_after();
       if (elect_one()) {
         if (has_g1) batch(j, cuda::std::true_type{});
         else batch(j, cuda::std::false_type{});
       }
       __syncwarp();
-      if (lane == 0) TRACE(j, 5);
     }
     if (elect_one()) tc_commit(bar(BAR_DONE));
     __syncwarp();
@@ -546,10 +469,8 @@ glm_bernoulli_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
       const int sx = it % SX, ux = it / SX;
       const int st = it % kStagesT, ut = it / kStagesT;
       mbar_wait(bar(BAR_XFULL + sx), ux & 1);
-      if (r == 0) TRACE(it, 6);
       mbar_wait(bar(BAR_TEMPTY + st), (ut & 1) ^ 1);           // GEMM 2 of tile it-3 released X^T[st]
-      if (r == 0) TRACE(it, 7);
-      if (LM == 2) mbar_wait(bar(BAR_LEMPTY + (it & 1)), ((it >> 1) & 1) ^ 1);
+      if (SPLIT_X) mbar_wait(bar(BAR_LEMPTY + (it & 1)), ((it >> 1) & 1) ^ 1);
       float4* xhi = reinterpret_cast<float4*>(sm + L::OFF_X + sx * kTile);
       float4* xlo = reinterpret_cast<float4*>(sm + L::OFF_XLO + (it & 1) * kTile);
       float* xt = reinterpret_cast<float*>(sm + L::OFF_XT + st * kXtStage + kb * kXtBlock);
@@ -561,7 +482,7 @@ glm_bernoulli_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
         const int idx = r * 8 + (c ^ (r & 7));      // 16-byte chunk holding d = 4c .. 4c+3 of row r
         const float4 v = xhi[idx];
         float x[4] = {v.x, v.y, v.z, v.w};
-        if (LM == 2) {
+        if (SPLIT_X) {
           float4 h, l;
           h.x = tf32_trunc(v.x); h.y = tf32_trunc(v.y); h.z = tf32_trunc(v.z); h.w = tf32_trunc(v.w);
           l.x = v.x - h.x; l.y = v.y - h.y; l.z = v.z - h.z; l.w = v.w - h.w;
@@ -574,26 +495,15 @@ glm_bernoulli_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
           for (int q = 0; q < 4; ++q) x[q] = tf32_rn(x[q]);
           xhi[idx] = make_float4(x[0], x[1], x[2], x[3]);
         }
-        if (BF) {
-          // natural layout, bf16: columns 4c .. 4c+3 of row r -> 8 bytes inside 16-byte chunk c/2
-          __nv_bfloat162 lo2 = __floats2bfloat162_rn(v.x, v.y), hi2 = __floats2bfloat162_rn(v.z, v.w);
-          uint2 pk;
-          pk.x = *reinterpret_cast<uint32_t*>(&lo2);
-          pk.y = *reinterpret_cast<uint32_t*>(&hi2);
-          *reinterpret_cast<uint2*>(sm + L::OFF_XT + st * kXtStage + r * 128 + (((c >> 1) ^ (r & 7)) << 4) +
-                                    (c & 1) * 8) = pk;
-        } else {
 #pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            const int d = c * 4 + q;
-            // X^T[d][n = r]: row d of k-block kb, 16-byte chunk (lane >> 2) ^ (d & 7), element lane & 3
-            xt[d * 32 + (((((r & 31) >> 2) ^ (d & 7)) << 2) | (r & 3))] = x[q];
-          }
+        for (int q = 0; q < 4; ++q) {
+          const int d = c * 4 + q;
+          // X^T[d][n = r]: row d of k-block kb, 16-byte chunk (lane >> 2) ^ (d & 7), element lane & 3
+          xt[d * 32 + (((((r & 31) >> 2) ^ (d & 7)) << 2) | (r & 3))] = x[q];
         }
       }
       fence_proxy_async();
       mbar_arrive(bar(BAR_XREADY + sx));
-      if (r == 0) TRACE(it, 8);
     }
   } else {
     // =========================== epilogue warps ========================================================
@@ -616,10 +526,8 @@ glm_bernoulli_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
       const int64_t row0 = (blockIdx.x + (int64_t)it * gridDim.x) * kRows;
       // GEMM 2 of tile it-2 (long finished) has released g^T[b]
       mbar_wait(bar(BAR_GEMPTY + b), (v & 1) ^ 1);
-      if (ew == 0 && lane == 0) TRACE(it, 11);
       // d1_full implies the split pass of this tile ran (x_ready -> GEMM 1 -> d1_full): y[st] is in place
       mbar_wait(bar(BAR_D1FULL + b), v & 1);
-      if (ew == 0 && lane == 0) TRACE(it, 9);
       tc_fence_after();
       uint32_t lr[kEpiCols];
       const uint32_t taddr = tmem + ((uint32_t)(sub * 32) << 16) + kColD1 + (uint32_t)b * 64u +
@@ -637,38 +545,27 @@ glm_bernoulli_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
       asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
       tc_fence_before();
       mbar_arrive(bar(BAR_D1EMPTY + b));            // D1[b] is in registers now
-      if (ew == 0 && lane == 0) TRACE(it, 10);
       uint8_t* gt = sm + L::OFF_G + b * kGBuf;
       if (row0 + kRows <= N) {
 #pragma unroll
         for (int j0 = 0; j0 < kEpiCols; j0 += 8) {
           float g[8];
-          epi_batch<false, 8, BF>(lr + j0, y, 1.f, acc + j0, g);
-          if (BF) store_g_bf16(gt, r, part * (kEpiCols / 8) + (j0 >> 3), g);
-          else {
+          epi_batch<false, 8>(lr + j0, y, 1.f, acc + j0, g);
 #pragma unroll
-            for (int j = 0; j < 8; ++j) *reinterpret_cast<float*>(gt + gofs[j] + (j0 + j) * 128) = g[j];
-          }
+          for (int j = 0; j < 8; ++j) *reinterpret_cast<float*>(gt + gofs[j] + (j0 + j) * 128) = g[j];
         }
       } else {
         const float vw = (row0 + r < N) ? 1.f : 0.f;
 #pragma unroll
         for (int j0 = 0; j0 < kEpiCols; j0 += 8) {
           float g[8];
-          epi_batch<true, 8, BF>(lr + j0, y, vw, acc + j0, g);
-          if (BF) store_g_bf16(gt, r, part * (kEpiCols / 8) + (j0 >> 3), g);
-          else {
+          epi_batch<true, 8>(lr + j0, y, vw, acc + j0, g);
 #pragma unroll
-            for (int j = 0; j < 8; ++j) *reinterpret_cast<float*>(gt + gofs[j] + (j0 + j) * 128) = g[j];
-          }
+          for (int j = 0; j < 8; ++j) *reinterpret_cast<float*>(gt + gofs[j] + (j0 + j) * 128) = g[j];
         }
       }
       fence_proxy_async();
       mbar_arrive(bar(BAR_GFULL + b));
-      if (ew == 0 && lane == 0) TRACE(it, 12);
-      if (ew == 4 && lane == 0) TRACE(it, 13);
-      if (ew == 3 && lane == 0) TRACE(it, 14);
-      if (ew == 15 && lane == 0) TRACE(it, 15);
     }
     // ---- CTA results: dW, db from TMEM; lp sums through shared memory (fixed order) ---------------------
     mbar_wait(bar(BAR_DONE), 0);
@@ -685,7 +582,7 @@ glm_bernoulli_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
       for (int d = 0; d < 32; ++d) dwf[d] = 0.f;
       const uint32_t t2 = tmem + ((uint32_t)(sub * 32) << 16);
 #pragma unroll
-      for (int kb = 0; kb < (BF ? 1 : 4); ++kb) {
+      for (int kb = 0; kb < 4; ++kb) {
         uint32_t dw[32], dbv[8];
         asm volatile(
             "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
@@ -696,7 +593,7 @@ glm_bernoulli_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
               "=r"(dw[14]), "=r"(dw[15]), "=r"(dw[16]), "=r"(dw[17]), "=r"(dw[18]), "=r"(dw[19]), "=r"(dw[20]),
               "=r"(dw[21]), "=r"(dw[22]), "=r"(dw[23]), "=r"(dw[24]), "=r"(dw[25]), "=r"(dw[26]), "=r"(dw[27]),
               "=r"(dw[28]), "=r"(dw[29]), "=r"(dw[30]), "=r"(dw[31])
-            : "r"(t2 + kColD2 + (uint32_t)kb * 40u)      // BF: one accumulator, dW in columns 0..31, db in 32
+            : "r"(t2 + kColD2 + (uint32_t)kb * 40u)
             : "memory");
         asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
                      : "=r"(dbv[0]), "=r"(dbv[1]), "=r"(dbv[2]), "=r"(dbv[3]), "=r"(dbv[4]), "=r"(dbv[5]),
@@ -760,7 +657,7 @@ int glm_tc_grid_x(int64_t N) {
 
 // returns 0 on success, a negative B2_ERR code when the TMA path cannot be used for these operands
 int launch_glm_tc(const float* X, const float* y, const float* W, const float* b, int64_t N, int P,
-                  float* partials, int gx, int mode, cudaStream_t s) {
+                  float* partials, int gx, bool split_x, cudaStream_t s) {
   using namespace tc;
   EncodeTiledFn enc = encode_fn();
   if (enc == nullptr) return B2_ERR_LAUNCH;
@@ -789,28 +686,17 @@ int launch_glm_tc(const float* X, const float* y, const float* W, const float* b
   }
   static bool attr_set = false;
   if (!attr_set) {
-    cudaFuncSetAttribute(glm_bernoulli_tc_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                         (int)Layout<0>::kSmemBytes);
-    cudaFuncSetAttribute(glm_bernoulli_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                         (int)Layout<1>::kSmemBytes);
-    cudaFuncSetAttribute(glm_bernoulli_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                         (int)Layout<2>::kSmemBytes);
-    cudaFuncSetAttribute(glm_bernoulli_tc_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                         (int)Layout<3>::kSmemBytes);
+    cudaFuncSetAttribute(glm_bernoulli_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                         (int)Layout<false>::kSmemBytes);
+    cudaFuncSetAttribute(glm_bernoulli_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                         (int)Layout<true>::kSmemBytes);
     attr_set = true;
   }
   dim3 grid((unsigned)gx, (unsigned)((P + kP - 1) / kP), 1);
-  // B2_GLM_TC_TRACE = device address (decimal) of a 64 x 16 int64 buffer for the event trace of CTA 0
-  const char* tr_env = getenv("B2_GLM_TC_TRACE");
-  long long* trace = tr_env ? reinterpret_cast<long long*>(strtoull(tr_env, nullptr, 10)) : nullptr;
-  if (mode == 3)
-    launch_pdl(glm_bernoulli_tc_kernel<3>, grid, dim3(kThreads), (size_t)Layout<3>::kSmemBytes, s, mx, my, W, b, N, P, partials, trace);
-  else if (mode == 2)
-    launch_pdl(glm_bernoulli_tc_kernel<2>, grid, dim3(kThreads), (size_t)Layout<2>::kSmemBytes, s, mx, my, W, b, N, P, partials, trace);
-  else if (mode == 1)
-    launch_pdl(glm_bernoulli_tc_kernel<1>, grid, dim3(kThreads), (size_t)Layout<1>::kSmemBytes, s, mx, my, W, b, N, P, partials, trace);
+  if (split_x)
+    launch_pdl(glm_bernoulli_tc_kernel<true>, grid, dim3(kThreads), (size_t)Layout<true>::kSmemBytes, s, mx, my, W, b, N, P, partials);
   else
-    launch_pdl(glm_bernoulli_tc_kernel<0>, grid, dim3(kThreads), (size_t)Layout<0>::kSmemBytes, s, mx, my, W, b, N, P, partials, trace);
+    launch_pdl(glm_bernoulli_tc_kernel<false>, grid, dim3(kThreads), (size_t)Layout<false>::kSmemBytes, s, mx, my, W, b, N, P, partials);
   return 0;
 }
 

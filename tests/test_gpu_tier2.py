@@ -274,9 +274,7 @@ def test_unchanged_logistic_model_d32_matches_oracle_trajectory():
         assert torch.allclose(got[k].detach().cpu().reshape(-1), cons[k].reshape(-1), atol=2e-4), k
 
 
-@pytest.mark.parametrize("flag_name,tol_sum,tol_g", [("default", 2e-5, 2e-4), ("B2_FLAG_GLM_3XTF32", 2e-5, 2e-4),
-                                                     ("B2_FLAG_GLM_BF16_GRAD", 2e-5, 2e-4),
-                                                     ("B2_FLAG_GLM_TF32", 5e-4, 2e-3)])
+@pytest.mark.parametrize("flag_name,tol_sum,tol_g", [("default", 2e-5, 2e-4), ("B2_FLAG_GLM_3XTF32", 2e-5, 2e-4)])
 def test_glm_kernel_full_size_against_oracle(flag_name, tol_sum, tol_g):
     """BASELINE size (N = 1e6, D = 32, P = 64): per-particle sums, dW and db of the tcgen05 kernel against
     the oracle's fp64 Bernoulli log-density (oracle/dists.py) differentiated by autograd on the CPU.
@@ -323,16 +321,20 @@ def test_glm_kernel_full_size_against_oracle(flag_name, tol_sum, tol_g):
     assert torch.equal(sum_p, sum2)
 
 
-@pytest.mark.parametrize("n,P,bias,flag", [(1, 1, True, "B2_FLAG_GLM_3XTF32"), (127, 3, False, "B2_FLAG_GLM_3XTF32"),
-                                           (128, 64, True, "B2_FLAG_GLM_3XTF32"), (129, 65, True, "B2_FLAG_GLM_3XTF32"),
-                                           (1, 1, True, None), (5000, 130, False, None),
-                                           (8192, 64, True, None), (70001, 64, True, None), (65535, 130, False, None)])
-def test_glm_tc_kernel_ragged_shapes_against_oracle(n, P, bias, flag):
+@pytest.mark.parametrize("n,P,bias,flag,y_offset", [
+    (1, 1, True, "B2_FLAG_GLM_3XTF32", 0), (127, 3, False, "B2_FLAG_GLM_3XTF32", 0),
+    (128, 64, True, "B2_FLAG_GLM_3XTF32", 0), (129, 65, True, "B2_FLAG_GLM_3XTF32", 0),
+    (1, 1, True, None, 0), (5000, 130, False, None, 0),
+    (8192, 64, True, None, 0), (70001, 64, True, None, 0), (65535, 130, False, None, 0),
+    (20000, 64, True, None, 4)])
+def test_glm_tc_kernel_ragged_shapes_against_oracle(n, P, bias, flag, y_offset):
     """Edge cases of the tiled kernel: a single row, one row short of / one past a 128-row tile, ragged
     particle slabs (65, 130), no bias.  With an explicit tensor-core flag the tcgen05 kernel runs at any
     size and its gradient contraction is single-pass TF32 on round-to-nearest operands: the tolerance is
     2^-11 of the LARGEST TERM budget (5e-4 x scale) for tiny N, where nothing averages; the default
-    dispatch (flag None: exact fp32 SIMT below 8 Ki rows, tcgen05 above) must meet the fp32 tolerances."""
+    dispatch (flag None: exact fp32 SIMT below 8 Ki rows, tcgen05 above) must meet the fp32 tolerances.
+    y_offset: y starts that many bytes past a 16-byte boundary, which TMA cannot load; such a y takes the
+    fp32 SIMT kernel at any size."""
     if EMULATE:
         pytest.skip("kernel test")
     from pyro_b200 import _native as N
@@ -346,7 +348,9 @@ def test_glm_tc_kernel_ragged_shapes_against_oracle(n, P, bias, flag):
     s_ref = od.bernoulli_logits(y.double(), logits).sum(1)
     g = y.double() - torch.sigmoid(logits)
     gW, gb = g @ X.double(), g.sum(1)
-    Xg, yg, Wg = X.to(DEV), y.to(DEV), W.to(DEV)
+    Xg, Wg = X.to(DEV), W.to(DEV)
+    yg = torch.cat([torch.zeros(y_offset // 4), y]).to(DEV)[y_offset // 4:]
+    assert yg.data_ptr() % 16 == y_offset
     bg = b.to(DEV) if bias else None
     sum_p = torch.empty(P, device=DEV)
     dW = torch.empty(P, D, device=DEV)

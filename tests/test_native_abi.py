@@ -40,6 +40,15 @@ def test_argument_validation_without_gpu():
                            None, 0, None) == -4
     assert L.b2_glm_bernoulli_logits(None, None, None, None, 10, 32, 8, 1.0, 1.0, 1.0, 0, None, None,
                                      None, None, None, 0, None) == -4
+    # retired GLM flag bits (8, 16, 64) and unknown bits are refused; the supported ones get as far as the
+    # workspace check (no workspace given).  The pointers are 16-byte aligned and never dereferenced.
+    x = ctypes.c_void_p(4096)
+    for bit in (8, 16, 64, 128):
+        assert L.b2_glm_bernoulli_logits(x, x, x, None, 10, 32, 8, 1.0, 1.0, 1.0, bit, None, None,
+                                         None, None, None, 0, None) == -2, bit
+    ok = N.B2_FLAG_ACCUMULATE_SUM | N.B2_FLAG_GLM_FP32 | N.B2_FLAG_GLM_3XTF32
+    assert L.b2_glm_bernoulli_logits(x, x, x, None, 10, 32, 8, 1.0, 1.0, 1.0, ok, None, None,
+                                     None, None, None, 0, None) == -5
     assert L.b2_nuts_small(None, None, None, None, None, None, 1, 1, 10, 1000.0, 0, None, None, None,
                            None, None, None, None) == -4
 
